@@ -153,6 +153,19 @@ class StdoutGuard:
         return False
 
 
+def dump_outputs(path, **arrays):
+    """--dump-outputs: what the last timed step returned, so that the outputs of two builds on the same seeded inputs
+    can be compared file for file.  Every file holds finite float32 values: <name>.npy the array with its non-finite
+    entries set to 0, <name>_nonfinite.npy which entries those were (0 finite, 1 NaN, 2 +inf, 3 -inf).  A tree that
+    divides by zero anywhere has a NaN fitness, as in the reference; with 0 among the constants many trees do."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float32)
+        kind = np.select([np.isnan(a), a == np.inf, a == -np.inf], [1, 2, 3], 0).astype(np.float32)
+        np.save(os.path.join(path, name + ".npy"), np.where(kind == 0, a, np.float32(0)).astype(np.float32))
+        np.save(os.path.join(path, name + "_nonfinite.npy"), kind)
+
+
 def descriptor_args(w, max_layer_cnt=None):
     return dict(max_tree_len=w["L"], input_len=w["V"], output_len=w["O"], using_funcs=FUNCS,
                 max_layer_cnt=max_layer_cnt or w["max_layer_cnt"], const_samples=CONSTS)
@@ -310,6 +323,8 @@ def run_reference(args, out):
     e1.record()
     torch.cuda.synchronize()
     sampler.active = False
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, fitness=fit.cpu().numpy())
     total_ms = e0.elapsed_time(e1)
     value = P * N * args.steps / (total_ms * 1e-3)
     check = float(torch.nan_to_num(fit, nan=0.0, posinf=0.0, neginf=0.0).clamp(max=1e6).mean())
@@ -613,11 +628,13 @@ def run_ours(args, out):
     ev_t0.record()
     for i in range(args.steps):
         abi.evogp_eval_set_timing_events(ctypes.c_void_p(kev[i][0].cuda_event), ctypes.c_void_p(kev[i][1].cuda_event))
-        step(i)
+        fit = step(i)
     ev_t1.record()
     torch.cuda.synchronize()
     t_wall = time.perf_counter() - t_wall0
     sampler.active = False
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, fitness=fit.cpu().numpy())     # N > 1: the exchanged fitness of the whole population
     abi.evogp_eval_set_timing_events(None, None)
     kern_ms = [a.elapsed_time(b) for a, b in kev]
     launches = _native.launch_count() - launches0
@@ -735,7 +752,10 @@ def main():
     ap.add_argument("--config", type=int, default=0, choices=[0, 2, 3], help="0: configs[1] at --gpus 1, configs[2] strong-scaled otherwise")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg (profiling runs)")
     ap.add_argument("--quick", action="store_true", help="skip the extra legs (config-5 loop, HBM kernels, config 3 on one GPU)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the fitness the last timed step computed to DIR/fitness.npy (finite values) and DIR/fitness_nonfinite.npy (which were NaN / inf)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     with StdoutGuard() as out:
         if args.impl == "reference":
             run_reference(args, out)

@@ -1,11 +1,13 @@
 #!/usr/bin/env python
-"""Runs the UNMODIFIED reference front-end (baseline/_ref/evogp: its Forest / GeneticProgramming / operators /
-SymbolicRegression python code) on a seeded GP loop and dumps every generation.
-    python tests/dropin_run.py reference out.npz   # over the reference's own extension (evogp/evogp_cuda*.so)
-    python tests/dropin_run.py ours out.npz        # over this repo's operator library (evogp_b200/lib/evogp_cuda_ops.so)
+"""Runs a seeded GP loop written against the EvoGP python API (Forest / GeneticProgramming / operators /
+SymbolicRegression) and dumps every generation.
+    python tests/dropin_run.py reference out.npz   # the reference's UNMODIFIED package (baseline/_ref/evogp) over its own extension
+    python tests/dropin_run.py ours out.npz        # the reference's package over this repo's operator library (evogp_cuda_ops.so)
+    python tests/dropin_run.py shim out.npz        # this repo's `evogp` import shim: its own front-end and operator library
 In `ours` mode the only thing replaced is the module `evogp.evogp_cuda` that evogp/tree/__init__.py:2 imports: a stub
 whose import registered torch.ops.evogp_cuda.* from this repo instead — the swap INTEGRATION.md describes.
-Spawned by tests/test_dropin.py (-m gpu)."""
+Populations are dumped as SHA-256 digests of their valid prefixes; fitness and forward outputs as values."""
+import hashlib
 import os
 import sys
 import types
@@ -27,16 +29,17 @@ def main():
         from evogp_b200 import _native
         _native.load_ops()                                  # TORCH_LIBRARY(evogp_cuda) from evogp_cuda_ops.so
         sys.modules["evogp.evogp_cuda"] = types.ModuleType("evogp.evogp_cuda")
-    sys.path.insert(0, REF)
+    front = ROOT if mode == "shim" else REF
+    sys.path.insert(0, front)
     import evogp
     import evogp.tree as rt
-    assert os.path.realpath(evogp.__file__).startswith(os.path.realpath(REF)), evogp.__file__
+    assert os.path.realpath(evogp.__file__).startswith(os.path.realpath(front)), evogp.__file__
     from evogp.algorithm import DefaultCrossover, DefaultMutation, DefaultSelection, GeneticProgramming
     from evogp.problem import SymbolicRegression
 
     loaded = [l.split()[-1] for l in open("/proc/self/maps") if "evogp" in l and l.rstrip().endswith(".so")]
     native = sorted(set(os.path.basename(p) for p in loaded))
-    if mode == "ours":
+    if mode != "reference":
         assert "evogp_cuda_ops.so" in native and not any(n.startswith("evogp_cuda.cpython") for n in native), native
     else:
         assert any(n.startswith("evogp_cuda.cpython") for n in native) and "libevogp_b200.so" not in native, native
@@ -64,9 +67,9 @@ def main():
         sel = selector.evaluate(f)
         lens = f.batch_subtree_size[:, 0].long()
         valid = (torch.arange(f.max_tree_len, device="cuda")[None, :] < lens[:, None])
-        dump[f"value{g}"] = torch.where(valid, f.batch_node_value, torch.zeros_like(f.batch_node_value)).cpu().numpy()
-        dump[f"type{g}"] = torch.where(valid, f.batch_node_type, torch.zeros_like(f.batch_node_type)).cpu().numpy()
-        dump[f"size{g}"] = torch.where(valid, f.batch_subtree_size, torch.zeros_like(f.batch_subtree_size)).cpu().numpy()
+        for name, a in (("value", f.batch_node_value), ("type", f.batch_node_type), ("size", f.batch_subtree_size)):
+            prefixes = torch.where(valid, a, torch.zeros_like(a)).cpu().numpy()
+            dump[f"{name}{g}"] = np.array(hashlib.sha256(prefixes.tobytes()).hexdigest())
         dump[f"fitness{g}"] = fit.cpu().numpy()
         dump[f"torch_fitness{g}"] = sel.cpu().numpy()
         sel = torch.where(torch.isnan(sel), torch.full_like(sel, float("-inf")), sel)     # pipeline/standard.py:43

@@ -1,6 +1,7 @@
 """Helpers for the -m gpu tests: call the C ABI (include/evogp_b200.h) through ctypes with torch
-device pointers, and move oracle/numpy data to the GPU."""
+device pointers, move oracle/numpy data to the GPU, and replay the reference's recorded results."""
 import ctypes as C
+import hashlib
 
 import numpy as np
 import torch
@@ -113,3 +114,81 @@ def assert_close_fitness(got, want, rtol=1e-5, atol=0.0, what=""):
     bad = err > tol
     assert not bad.any(), (f"{what}: {bad.sum()} of {m.sum()} beyond rtol={rtol}; worst rel "
                            f"{(err[bad] / np.maximum(np.abs(want[m][bad]), 1e-30)).max():.3e}")
+
+
+def _host(a):
+    return np.ascontiguousarray(a.cpu().numpy() if isinstance(a, torch.Tensor) else a)
+
+
+def prefix_digest(v, t, s):
+    """SHA-256 of a forest's valid prefixes (row tails zeroed, each row's length from its own size[:, 0]): two forests
+    have the same digest when their prefixes agree bit for bit."""
+    v, t, s = _host(v), _host(t), _host(s)
+    L = v.shape[1]
+    valid = np.arange(L)[None, :] < np.clip(s[:, 0].astype(np.int64), 0, L)[:, None]
+    h = hashlib.sha256()
+    for a in (v.view(np.uint32), t, s):
+        h.update(np.where(valid, a, 0).astype(a.dtype).tobytes())
+    return h.hexdigest()
+
+
+def call_key(op, *args):
+    """Digest of an operator name and its inputs (arrays by dtype, shape and bytes; scalars by value)."""
+    h = hashlib.sha256(op.encode())
+    for a in args:
+        if isinstance(a, (torch.Tensor, np.ndarray)):
+            a = _host(a)
+            h.update(f"{a.dtype.str}{a.shape}".encode())
+            h.update(a.tobytes())
+        else:
+            h.update(repr(a).encode())
+    return h.hexdigest()
+
+
+class GoldenReference:
+    """The reference's own CUDA kernels (forward.cu / generate.cu / mutation.cu compiled unmodified), replayed from
+    results recorded on a B200 (tests/golden/make_golden.py parity).  Each result is stored under call_key of its
+    inputs, so a test whose inputs changed finds no result rather than a wrong one.  Fitness and evaluation results
+    are stored as values; the tree producers, whose outputs are too large to store, as prefix_digest of their output."""
+
+    def __init__(self, path):
+        with np.load(path) as f:
+            self.results = {k: f[k] for k in f.files}
+
+    def _get(self, *call):
+        key = call_key(*call)
+        assert key in self.results, f"no recorded reference result for these {call[0]} inputs (key {key[:16]})"
+        r = self.results[key]
+        return str(r) if r.dtype.kind == "U" else r
+
+    def generate(self, pop, gp_len, var_len, out_len, out_prob, const_prob, keys, depth2leaf, roulette, const_samples):
+        return self._get("generate", pop, gp_len, var_len, out_len, out_prob, const_prob, keys, depth2leaf, roulette, const_samples)
+
+    def crossover(self, value, ntype, size, left_idx, right_idx, left_node, right_node):
+        return self._get("crossover", value, ntype, size, left_idx, right_idx, left_node, right_node)
+
+    def mutate(self, value, ntype, size, mut_idx, nvalue, ntype_new, nsize):
+        return self._get("mutate", value, ntype, size, mut_idx, nvalue, ntype_new, nsize)
+
+    def sr_fitness(self, value, ntype, size, variables, labels, use_mse=True, kernel_type=4):
+        return self._get("sr_fitness", value, ntype, size, variables, labels, bool(use_mse), kernel_type)
+
+    def evaluate(self, value, ntype, size, variables, out_len):
+        return self._get("evaluate", value, ntype, size, variables, out_len)
+
+
+class RecordingReference(GoldenReference):
+    """Runs the reference's kernels (oracle.ref_gpu()) and records what GoldenReference replays."""
+
+    def __init__(self, live):
+        self.live, self.results = live, {}
+
+    def _get(self, op, *args):
+        out = getattr(self.live, op)(*args)
+        torch.cuda.synchronize()
+        r = np.array(prefix_digest(*out)) if isinstance(out, tuple) else out.cpu().numpy()
+        self.results[call_key(op, *args)] = r
+        return str(r) if r.dtype.kind == "U" else r
+
+    def save(self, path):
+        np.savez_compressed(path, **self.results)

@@ -1,24 +1,34 @@
 """-m gpu: parity of the sm_100a kernels, called through the C ABI, against
   (a) the CPU oracle (oracle/evogp_oracle.c) — bit-exact for integer/index work,
-  (b) the reference's own CUDA kernels compiled unmodified (oracle/_ref/libevogp_ref.so) —
-      bit-exact valid prefixes, fp32 fitness within 1e-5 relative (BASELINE.json north_star).
+  (b) the reference's own CUDA kernels compiled unmodified, as recorded on a B200 in tests/golden/ref_parity.npz
+      (tests/golden/make_golden.py parity) — bit-exact valid prefixes, fp32 fitness within 1e-5 relative
+      (BASELINE.json north_star).
 """
+import os
+
 import numpy as np
 import pytest
 import torch
 
 import gpu_util as G
-from conftest import (ALL_FUNCS, ARITH_FUNCS, EXACT_FUNCS, depth2leaf, make_data, make_forest, prefix_equal, roulette)
+from conftest import ALL_FUNCS, ARITH_FUNCS, EXACT_FUNCS, depth2leaf, make_data, make_forest, roulette
 
 pytestmark = pytest.mark.gpu
 RTOL = 1e-5   # north star: fp32 fitness within 1e-5 relative
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_parity.npz")
 
 
 @pytest.fixture(scope="module")
 def ref(orc):
-    if not orc.ref_gpu_available():
-        pytest.skip("oracle/_ref/libevogp_ref.so not built")
-    return orc.ref_gpu()
+    """The reference's results replayed from GOLDEN; with EVOGP_RECORD_REFERENCE=<path.npz> (make_golden.py parity)
+    its kernels run live from oracle/_ref and the results are written to that file instead."""
+    record = os.environ.get("EVOGP_RECORD_REFERENCE")
+    if not record:
+        yield G.GoldenReference(GOLDEN)
+        return
+    rec = G.RecordingReference(orc.ref_gpu())
+    yield rec
+    rec.save(record)
 
 
 def gen_args(funcs, layers, consts=(-1.0, 0.0, 1.0), leaf_prob=0.2):
@@ -52,11 +62,7 @@ def test_generate_bit_exact(native, orc, ref, case):
     torch.cuda.synchronize()
     for g, w in zip(got, want):
         assert G.same_bits(g, w)           # whole rows: oracle and kernel both zero-fill tails
-    rv, rt, rs = ref.generate(pop, L, V, O, 0.5, 0.5, k, a, r, c)
-    torch.cuda.synchronize()
-    lens = want[2][:, 0]
-    for g, w in zip(got, (rv, rt, rs)):
-        assert prefix_equal(g.cpu().numpy(), w.cpu().numpy(), lens)   # reference defines prefixes only
+    assert G.prefix_digest(*got) == ref.generate(pop, L, V, O, 0.5, 0.5, k, a, r, c)   # reference defines prefixes only
     orc.check_forest(*[g.cpu().numpy() for g in got], input_len=V, output_len=O)
 
 
@@ -84,10 +90,7 @@ def test_crossover_bit_exact(native, orc, ref, pop, L, funcs, layers, n_new):
     torch.cuda.synchronize()
     for g, w in zip(got, want):
         assert G.same_bits(g, w)
-    rgot = ref.crossover(*df, *di)
-    torch.cuda.synchronize()
-    for g, w in zip(got, rgot):
-        assert prefix_equal(g.cpu().numpy(), w.cpu().numpy(), want[2][:, 0])
+    assert G.prefix_digest(*got) == ref.crossover(*df, *di)
     orc.check_forest(*[g.cpu().numpy() for g in got], input_len=3)
     assert (want[2][:, 0] == lens[idx[0]]).sum() > n_new // 25      # fallbacks were exercised
 
@@ -107,10 +110,7 @@ def test_mutate_bit_exact(native, orc, ref, pop, L, layers):
     torch.cuda.synchronize()
     for g, w in zip(got, want):
         assert G.same_bits(g, w)
-    rgot = ref.mutate(*dargs)
-    torch.cuda.synchronize()
-    for g, w in zip(got, rgot):
-        assert prefix_equal(g.cpu().numpy(), w.cpu().numpy(), want[2][:, 0])
+    assert G.prefix_digest(*got) == ref.mutate(*dargs)
 
 
 # --------------------------------------------------------------------------- SR fitness
